@@ -66,6 +66,11 @@ SIGNATURES = {
     "danet_body_uv_losses_workspace_bytes": (c_i64, [c_int, c_int]),
     "danet_body_uv_losses": (c_int, [c_int, c_int, c_int, c_int, c_i64, c_i64, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p,
                                      c_p, c_f, c_f, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "danet_dp_uvia_losses_workspace_bytes": (c_i64, [c_int, c_int, c_int, c_int]),
+    "danet_dp_uvia_losses": (c_int, [c_int, c_int, c_int, c_int, c_int] + [c_p] * 12 + [c_int, c_f, c_f, c_f]
+                             + [c_p] * 7),
+    "danet_stn_kps_losses_workspace_bytes": (c_i64, [c_int, c_int]),
+    "danet_stn_kps_losses": (c_int, [c_int, c_int, c_int, c_p, c_p, c_f, c_p, c_p, c_p, c_p, c_p]),
     "danet_raster_create": (c_int, [ctypes.POINTER(RasterDesc), ctypes.POINTER(c_p)]),
     "danet_raster_destroy": (c_int, [c_p]),
     "danet_raster_workspace_bytes": (c_i64, [c_p, c_int]),

@@ -1,22 +1,34 @@
-"""Dense IUV losses of the training step (SURVEY section 8f-2) with the reference's call surface:
+"""IUV-branch losses of the training step (SURVEY section 8f-2) with the reference's call surface:
 
     loss_U, loss_V, loss_IndexUV, loss_segAnn = body_uv_losses(u_pred, v_pred, index_pred, ann_pred, uvia_list, has_iuv)
     loss_pU, loss_pV, loss_pIndexUV           = part_iuv_losses(part_iuv_pred, part_iuv_gt, has_iuv)
+    loss_Udp, loss_Vdp, loss_IndexUVdp, loss_segAnndp = dp_uvia_losses(u_pred, v_pred, index_pred, ann_pred,
+                                                                       **uvia_dp_gt, has_dp=has_dp)
+    loss_roi, stn_centers                     = stn_kps_losses(skps_hm_pred, smpl_kps_gt)
 
 `body_uv_losses` is models/danet/iuv_estimator.py:304-341; `part_iuv_losses` is the loop over the 24 part crops of
 iuv_estimator.py:232-255 as one launch.  Forward and backward are ONE fused CUDA pass (csrc/losses.cu,
 danet_body_uv_losses): the gradients w.r.t. the predictions are produced with the losses and handed to autograd by a
 torch.autograd.Function.  No CPU path.
 
-Deviation from the reference, stated: when no image has IUV ground truth the reference returns `torch.zeros(1)` per
-loss after a host synchronisation (`torch.sum(has_iuv) > 0`); here the losses are 0-dim zeros and nothing synchronises
-(the count stays on the device)."""
+`dp_uvia_losses` is iuv_estimator.py:343-419 with the has_dp selection of :106-121 (csrc/point_losses.cu,
+danet_dp_uvia_losses); `stn_kps_losses` is the soft-argmax of :137-140 with loss_roi of :159-171 (danet_stn_kps_losses).
+
+Deviations from the reference, stated:
+- when no image has IUV / DensePose ground truth the reference returns `torch.zeros(1)` per loss after a host
+  synchronisation (`torch.sum(has_iuv) > 0`); here the losses are 0-dim zeros and nothing synchronises (the count stays
+  on the device);
+- a DensePose part or annotation label outside its class range makes the reference raise (inside cross_entropy); here
+  the affected loss is NaN, because raising would need a host synchronisation."""
 import torch
 from torch.autograd.function import once_differentiable
 
 from . import _lib
 
 POINT_REGRESSION_WEIGHTS = 0.5                  # configs/danet_default.yaml:23 (cfg.DANET.POINT_REGRESSION_WEIGHTS)
+INDEX_WEIGHTS = 2.0                             # configs/danet_default.yaml:19 (cfg.DANET.INDEX_WEIGHTS)
+PART_WEIGHTS = 0.3                              # configs/danet_default.yaml:21 (cfg.DANET.PART_WEIGHTS)
+STN_KPS_WEIGHTS = 1.0                           # configs/danet_default.yaml:35 (cfg.DANET.STN_KPS_WEIGHTS)
 
 
 def _launch(N, C, Cann, HW, pred_stride, map_stride, u, v, idx, ann, U, V, I, A, has, batch_size, point_weight, dev,
@@ -146,3 +158,124 @@ def part_iuv_losses(part_iuv_pred, part_iuv_gt, has_iuv=None, point_weight=POINT
     has = _has_u8(has_iuv, part_iuv_pred.device, repeat=part_iuv_pred.shape[1])
     L = _PartIuvLosses.apply(part_iuv_pred, part_iuv_gt, has, point_weight)
     return L[0], L[1], L[2]
+
+
+class _DpUviaLosses(torch.autograd.Function):
+    """losses [4] = (loss_Udp, loss_Vdp, loss_IndexUVdp, loss_segAnndp) of the DensePose points; the backward multiplies
+    the gradients the fused pass already wrote by the incoming d/d losses[k]."""
+
+    @staticmethod
+    def forward(ctx, u, v, idx, ann, X, Y, I, Up, Vp, Wp, alab, has, align, weights):
+        dev = u.device
+        B, C, S = u.shape[0], u.shape[1], u.shape[2]
+        P = X.shape[1]
+        preds = [_f32(t, dev) for t in (u, v, idx, ann)]
+        pts = [_f32(t, dev) for t in (X, Y, I, Up, Vp, Wp, alab)]
+        grads = [torch.empty_like(t) if ctx.needs_input_grad[k] else None for k, t in enumerate(preds)]
+        lib = _lib.load()
+        with torch.cuda.device(dev):
+            ws = torch.empty(int(lib.danet_dp_uvia_losses_workspace_bytes(B, C, S, P)), dtype=torch.uint8, device=dev)
+            losses = torch.empty(4, device=dev)
+            _lib.check(lib.danet_dp_uvia_losses(B, C, ann.shape[1], S, P, *[_lib.ptr(t) for t in preds + pts], _lib.ptr(has),
+                                                int(align), *[float(w) for w in weights], _lib.ptr(losses),
+                                                *[_lib.ptr(g) for g in grads], _lib.ptr(ws), _lib.stream_ptr(dev)),
+                       "dp_uvia_losses")
+        ctx.grads = grads
+        ctx.dtypes = [t.dtype for t in (u, v, idx, ann)]
+        return losses
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        out = [None if t is None else (t * g[k]).to(ctx.dtypes[k]) for k, t in enumerate(ctx.grads)]
+        return (*out,) + (None,) * 10
+
+
+def dp_uvia_losses(U_estimated, V_estimated, Index_UV, Ann_Index, body_uv_X_points, body_uv_Y_points, body_uv_I_points,
+                   body_uv_Ind_points, body_uv_U_points, body_uv_V_points, body_uv_point_weights, body_uv_ann_labels,
+                   body_uv_ann_weights=None, has_dp=None, align_corners=False, index_weight=INDEX_WEIGHTS,
+                   part_weight=PART_WEIGHTS, point_weight=POINT_REGRESSION_WEIGHTS):
+    """models/danet/iuv_estimator.py:343-419 with the has_dp selection of :106-121 done on the device.
+    U_estimated / V_estimated / Index_UV [B,C,S,S], Ann_Index [B,Cann,S,S]; the DensePose targets with the reference's
+    keyword names: X / Y / I / Ind points [B,P], U / V points and point weights [B,C*P], ann labels [B,S*S];
+    has_dp [B] or None (every sample).  body_uv_Ind_points and body_uv_ann_weights are accepted and not used, as in the
+    reference.  align_corners=True samples like torch 1.1's grid_sample.  Returns (loss_Udp, loss_Vdp, loss_IndexUVdp,
+    loss_segAnndp), 0-dim, differentiable w.r.t. the four predictions."""
+    _lib.require_cuda(U_estimated, "U_estimated")
+    u = U_estimated
+    if u.dim() != 4 or u.shape[2] != u.shape[3] or V_estimated.shape != u.shape or Index_UV.shape != u.shape:
+        raise ValueError("dp_uvia_losses: U/V/Index predictions must share one [B,C,S,S] shape")
+    B, C, S = u.shape[0], u.shape[1], u.shape[2]
+    if Ann_Index.dim() != 4 or Ann_Index.shape[0] != B or Ann_Index.shape[2:] != u.shape[2:] or Ann_Index.shape[1] < 1:
+        raise ValueError("dp_uvia_losses: Ann_Index must be [B,Cann,S,S] like the predictions")
+    if body_uv_X_points.dim() != 2 or body_uv_X_points.shape[0] != B or body_uv_X_points.shape[1] < 1:
+        raise ValueError("dp_uvia_losses: body_uv_X_points must be [B,P] with P >= 1")
+    P = body_uv_X_points.shape[1]
+    for name, t in (("body_uv_Y_points", body_uv_Y_points), ("body_uv_I_points", body_uv_I_points),
+                    ("body_uv_Ind_points", body_uv_Ind_points)):
+        if tuple(t.shape) != (B, P):
+            raise ValueError("dp_uvia_losses: %s must be [B,P] = [%d,%d]" % (name, B, P))
+    for name, t in (("body_uv_U_points", body_uv_U_points), ("body_uv_V_points", body_uv_V_points),
+                    ("body_uv_point_weights", body_uv_point_weights)):
+        if t.shape[0] != B or t.numel() != B * C * P:
+            raise ValueError("dp_uvia_losses: %s must be [B,C*P] = [%d,%d]" % (name, B, C * P))
+    if body_uv_ann_labels.shape[0] != B or body_uv_ann_labels.numel() != B * S * S:
+        raise ValueError("dp_uvia_losses: body_uv_ann_labels must be [B,S*S] = [%d,%d]" % (B, S * S))
+    if has_dp is not None and tuple(has_dp.shape) != (B,):
+        raise ValueError("dp_uvia_losses: has_dp must have one entry per sample")
+    if B == 0 or C == 0 or S == 0:                                 # nothing to sum: zeros that still carry a graph
+        z = U_estimated.sum() * 0 + V_estimated.sum() * 0 + Index_UV.sum() * 0 + Ann_Index.sum() * 0
+        return z, z, z, z
+    flat = lambda t, n: t.reshape(B, n)
+    L = _DpUviaLosses.apply(U_estimated, V_estimated, Index_UV, Ann_Index, body_uv_X_points, body_uv_Y_points,
+                            body_uv_I_points, flat(body_uv_U_points, C * P), flat(body_uv_V_points, C * P),
+                            flat(body_uv_point_weights, C * P), flat(body_uv_ann_labels, S * S),
+                            _has_u8(has_dp, u.device), bool(align_corners), (index_weight, part_weight, point_weight))
+    return L[0], L[1], L[2], L[3]
+
+
+class _StnKpsLosses(torch.autograd.Function):
+    """(loss_roi [1], stn_centers [B,J,2]); the centres are not differentiable (every later use of them in the reference
+    is detached or thresholded)."""
+
+    @staticmethod
+    def forward(ctx, hm, kps, weight):
+        dev = hm.device
+        B, J, S = hm.shape[0], hm.shape[1], hm.shape[2]
+        h_, k_ = _f32(hm, dev), _f32(kps, dev)
+        grad = torch.empty_like(h_) if ctx.needs_input_grad[0] else None
+        lib = _lib.load()
+        with torch.cuda.device(dev):
+            ws = torch.empty(int(lib.danet_stn_kps_losses_workspace_bytes(B, J)), dtype=torch.uint8, device=dev)
+            loss = torch.empty(1, device=dev)
+            centers = torch.empty(B, J, 2, device=dev)
+            _lib.check(lib.danet_stn_kps_losses(B, J, S, _lib.ptr(h_), _lib.ptr(k_), float(weight), _lib.ptr(loss),
+                                                _lib.ptr(centers), _lib.ptr(grad), _lib.ptr(ws), _lib.stream_ptr(dev)),
+                       "stn_kps_losses")
+        ctx.grad = grad
+        ctx.dtype = hm.dtype
+        ctx.mark_non_differentiable(centers)
+        return loss, centers
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g, _g_centers):
+        if ctx.grad is None:
+            return None, None, None
+        return (ctx.grad * g[0]).to(ctx.dtype), None, None
+
+
+def stn_kps_losses(skps_hm_pred, smpl_kps_gt, weight=STN_KPS_WEIGHTS):
+    """iuv_estimator.py:137-140 and 159-171.  skps_hm_pred [B,J,S,S] (the key-point heat maps), smpl_kps_gt [B,J,3]
+    (x, y in [-1, 1], weight).  Returns (loss_roi 0-dim, differentiable w.r.t. skps_hm_pred; stn_centers [B,J,2] fp32,
+    x from columns and y from rows, not differentiable)."""
+    _lib.require_cuda(skps_hm_pred, "skps_hm_pred")
+    hm = skps_hm_pred
+    if hm.dim() != 4 or hm.shape[2] != hm.shape[3] or hm.shape[1] < 1:
+        raise ValueError("stn_kps_losses: skps_hm_pred must be [B,J,S,S]")
+    if tuple(smpl_kps_gt.shape) != (hm.shape[0], hm.shape[1], 3):
+        raise ValueError("stn_kps_losses: smpl_kps_gt must be [B,J,3] = [%d,%d,3]" % (hm.shape[0], hm.shape[1]))
+    if hm.shape[0] == 0 or hm.shape[2] == 0:
+        return hm.sum() * 0, torch.zeros(hm.shape[0], hm.shape[1], 2, device=hm.device)
+    loss, centers = _StnKpsLosses.apply(hm, smpl_kps_gt, weight)
+    return loss[0], centers

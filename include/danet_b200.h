@@ -117,6 +117,37 @@ int danet_body_uv_losses(int32_t N, int32_t C, int32_t Cann, int32_t HW, int64_t
                          danet_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * DensePose-point losses of the training step (SURVEY section 8f-2), forward and backward in one
+ * pass.  Replaces models/danet/iuv_estimator.py:343-419 (IUV_Estimator.dp_uvia_losses), the has_dp
+ * selection of iuv_estimator.py:106-121 and the autograd graph torch records for them.
+ * Predictions u/v/index [B,C,S,S], ann [B,Cann,S,S]; points X/Y/I [B,P] (pixel coordinates, part
+ * label); U/V/point_weights [B,C*P] (channel c of point p at c*P + p); ann_labels [B,S*S] (pixel
+ * h*S + w); labels are truncated like .to(int64); all fp32.  has_dp [B] uint8 or NULL (every sample).
+ * The maps are sampled bilinearly (zero padding) at grid (X - S/2) * 2/S, (Y - S/2) * 2/S with
+ * grid_sample's align_corners = `align_corners`.  losses[4] = { point_weight * sum w smooth_l1(w (u^ - U)),
+ * the same for v, part_weight * mean cross-entropy(index^, I) over the selected samples' B_sel*P points,
+ * index_weight * mean cross-entropy(ann, ann_labels) over their B_sel*S*S pixels } (all zero when no
+ * sample is selected; a label outside [0, C) / [0, Cann) makes its loss NaN).  grad_* (NULL to skip)
+ * receive d losses[k] / d prediction.  Deterministic (fixed summation order, no float atomics). */
+int64_t danet_dp_uvia_losses_workspace_bytes(int32_t B, int32_t C, int32_t S, int32_t P);
+int danet_dp_uvia_losses(int32_t B, int32_t C, int32_t Cann, int32_t S, int32_t P, const float* u_pred,
+                         const float* v_pred, const float* index_pred, const float* ann_pred, const float* X_points,
+                         const float* Y_points, const float* I_points, const float* U_points, const float* V_points,
+                         const float* point_weights, const float* ann_labels, const uint8_t* has_dp,
+                         int32_t align_corners, float index_weight, float part_weight, float point_weight,
+                         float* losses, float* grad_u, float* grad_v, float* grad_index, float* grad_ann,
+                         void* workspace, danet_stream_t stream);
+
+/* STN key-point loss (loss_roi) through the soft-argmax.  Replaces iuv_estimator.py:137-140 (centres:
+ * softmax_integral_tensor of 10 * map, utils/keypoints.py:334-394, / (S/2) - 1) and :159-171.  hm
+ * [B,J,S,S], kps_gt [B,J,3] (x, y in [-1, 1], weight).  loss[1] = weight * sum over joints with
+ * w != 0 of w * sum_xy smooth_l1(c - gt) / B; centers [B,J,2] (x from columns, y from rows);
+ * grad_hm (NULL to skip) = d loss / d hm.  Deterministic. */
+int64_t danet_stn_kps_losses_workspace_bytes(int32_t B, int32_t J);
+int danet_stn_kps_losses(int32_t B, int32_t J, int32_t S, const float* hm, const float* kps_gt, float weight,
+                         float* loss, float* centers, float* grad_hm, void* workspace, danet_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * IUV rasteriser.  Replaces utils/renderer.py:207-298 (IUV_Renderer) and the third-party
  * neural_renderer forward pass it calls; optionally fuses utils/iuvmap.py:103-151 (iuv_img2map).
  * ------------------------------------------------------------------------------------------ */
